@@ -4,6 +4,7 @@ one TRAINING step = forward + soft-target CE + backward + (DP gradient all-reduc
 parameters/activations (main.py:157), dropout active, synthetic images and random-init weights.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B] [--config vit_b16_224]
+                    [--dump-outputs DIR]
 
 N > 1: launched by the driver as `python -m torch.distributed.run --nproc-per-node N bench.py --gpus N ...`.
 Prints ONE JSON line on rank 0 (contract in the task statement): `value` = images/s over all GPUs with inputs resident
@@ -145,6 +146,41 @@ def build_oracle_model(c):
 def soft_targets(labels_a, labels_b, lam, classes):
     oh = torch.nn.functional.one_hot
     return lam * oh(labels_a, classes).float() + (1 - lam) * oh(labels_b, classes).float()
+
+
+DUMP_SAMPLE = 1 << 22          # elements kept of a larger array (16 MB in float32): four arrays stay under 64 MB
+
+
+def _host_sample(t):
+    """`t` as float32 on the host. Beyond DUMP_SAMPLE elements: the flattened tensor at DUMP_SAMPLE sorted positions
+    drawn from a fixed seed, so every run and every build of the same configuration keeps the same positions."""
+    t = t.detach()
+    if t.numel() > DUMP_SAMPLE:
+        idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.float().cpu()
+
+
+def step_outputs(logits, loss=None, model=None):
+    """What a caller of the timed step holds after its last step, copied to the host: the logits, and for a training
+    step the loss, the updated parameters and their gradients (each flattened and concatenated in model.parameters()
+    order; a parameter without a gradient contributes zeros)."""
+    out = {"logits": _host_sample(logits)}
+    if loss is not None:
+        out["loss"] = _host_sample(loss.reshape(1))
+    if model is not None:
+        params = list(model.parameters())
+        out["params"] = _host_sample(torch.cat([p.detach().float().reshape(-1) for p in params]))
+        out["grads"] = _host_sample(torch.cat([(torch.zeros_like(p) if p.grad is None else p.grad).float().reshape(-1)
+                                               for p in params]))
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
 
 
 def cpu_reference_throughput(c, steps, warmup, batch):
@@ -290,7 +326,7 @@ def run_torch_gpu_arm(args, c):
     res = {}
     for name, comp in (("eager", False), ("compiled_reduce_overhead", True)):
         try:
-            ips, ms = torch_gpu_throughput(c, device, B, max(3, args.steps), max(3, args.warmup), compiled=comp, infer=infer)
+            ips, ms = torch_gpu_throughput(c, device, B, args.steps, max(3, args.warmup), compiled=comp, infer=infer)
             res[name] = {"value": ips, "ms_per_step": ms}
         except Exception as e:                                        # e.g. no host compiler for inductor on the box
             res[name] = {"unavailable": f"{type(e).__name__}: {str(e)[:200]}"}
@@ -308,9 +344,9 @@ def run_reference_arm(args, c):
     batch = args.cpu_batch
     infer = args.mode == "infer"
     if infer:
-        ips, sec, threads, batch = cpu_reference_forward(c, max(1, args.steps), max(0, min(args.warmup, 1)), batch)
+        ips, sec, threads, batch = cpu_reference_forward(c, args.steps, max(0, min(args.warmup, 1)), batch)
     else:
-        ips, sec, threads = cpu_reference_throughput(c, max(1, args.steps), max(0, min(args.warmup, 1)), batch)
+        ips, sec, threads = cpu_reference_throughput(c, args.steps, max(0, min(args.warmup, 1)), batch)
     line = {
         "metric": metric_name(args.config, args.curve, infer), "value": ips, "unit": "images/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -402,6 +438,8 @@ def run_infer(args, c):
         e1.record()
         sync_all()
         clocks = sampler.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:                            # before the e2e replays overwrite static_out
+            write_outputs(args.dump_outputs, step_outputs(out))
         t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=device)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -425,7 +463,7 @@ def run_infer(args, c):
 
         for k in range(2):
             consumed[k].record()
-        e2e_steps = max(3, args.steps)
+        e2e_steps = args.steps
         sync_all()
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0.record()
@@ -615,7 +653,15 @@ def main():
                          "slower (profiles/r2_bench_2gpu_*.json: 32.86 vs 32.49 ms, exposed 1.02 vs 0.61 ms): the persistent "
                          "one-CTA-per-SM kernels leave NCCL no SM to run on, and its CTAs then delay the next kernel's wave")
     ap.add_argument("--no-exposed", action="store_true", help="N > 1: skip the second (collective-free) capture that measures allreduce_exposed_ms")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32): logits, and for --mode train "
+                         "also loss, params and grads; arrays above 4 Mi elements are a fixed seeded sample. Inputs are "
+                         "seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     c = dict(CONFIGS[args.config])
     if args.config == "vit_b16_1024":
         args.mode = "infer"                                           # 4096-token config is an inference sweep
@@ -665,9 +711,12 @@ def main():
     lb = torch.randint(0, classes, (B,), generator=g, device=device)
     tgt = soft_targets(la, lb, 0.3, classes)
 
+    eager_logits = [None]                                             # detached: no autograd graph outlives the step
+
     def eager_step(images):
         opt.zero_grad(set_to_none=True)
         logits = model(images)
+        eager_logits[0] = logits.detach()
         loss = crit(logits, tgt)
         loss.backward()
         opt.step()                                                    # all-reduce (N > 1) + clip + AdamW, fused
@@ -731,6 +780,9 @@ def main():
     ms_local = e0.elapsed_time(e1)
     launches = (ops.LAUNCHES - launches0) if graphed is None else launches_per_step * args.steps
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:                                # before the e2e steps train the model further
+        logits = eager_logits[0] if graphed is None else graphed.logits
+        write_outputs(args.dump_outputs, step_outputs(logits, loss, model))
     t = torch.tensor([ms_local], dtype=torch.float64, device=device)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -784,7 +836,7 @@ def main():
 
     for s in range(2):
         consumed[s].record()
-    e2e_steps = max(3, args.steps)
+    e2e_steps = args.steps
     sync_all()
     t0 = torch.cuda.Event(enable_timing=True); t1 = torch.cuda.Event(enable_timing=True)
     t0.record()

@@ -57,11 +57,10 @@ def _compile(src, obj, verbose):
     return r.stderr
 
 
-def build(force=False, verbose=False):
-    os.makedirs(OBJ_DIR, exist_ok=True)
-    os.makedirs(LIB_DIR, exist_ok=True)
-    # staleness by CONTENT hash (source + every header + flags), not mtime: the tree is copied to the GPU box with fresh
-    # timestamps, and a spurious rebuild there would burn GPU-box minutes
+def _plan(force=False):
+    """-> (compile jobs, every object, objects of deleted sources). Reads only, so it works in a read-only tree."""
+    # staleness by CONTENT hash (source + every header + flags), not mtime: a copied or freshly checked-out tree has new
+    # timestamps, and a spurious rebuild would cost minutes
     srcs = sorted(glob.glob(os.path.join(CSRC, "*.cu")))
     hdrs = _headers()
     flags = " ".join(FLAGS)
@@ -72,6 +71,20 @@ def build(force=False, verbose=False):
         want = _sha([s] + hdrs, flags)
         if force or not os.path.exists(o) or _stamp(o + ".sha") != want:
             jobs.append((s, o, want))
+    stale = [o for o in glob.glob(os.path.join(OBJ_DIR, "*.o")) if o not in objs]      # objects of deleted sources
+    return jobs, objs, stale
+
+
+def up_to_date():
+    """True when build() would compile and link nothing."""
+    jobs, _objs, stale = _plan()
+    return not jobs and not stale and os.path.exists(LIB)
+
+
+def build(force=False, verbose=False):
+    os.makedirs(OBJ_DIR, exist_ok=True)
+    os.makedirs(LIB_DIR, exist_ok=True)
+    jobs, objs, stale = _plan(force)
     if jobs:
         with cf.ThreadPoolExecutor(max_workers=min(8, len(jobs))) as ex:
             futs = {ex.submit(_compile, s, o, verbose): (o, want) for s, o, want in jobs}
@@ -82,7 +95,6 @@ def build(force=False, verbose=False):
                     fh.write(want)
                 if verbose:
                     sys.stderr.write(log)
-    stale = [o for o in glob.glob(os.path.join(OBJ_DIR, "*.o")) if o not in objs]      # objects of deleted sources
     for o in stale:
         os.remove(o)
     if jobs or stale or not os.path.exists(LIB):

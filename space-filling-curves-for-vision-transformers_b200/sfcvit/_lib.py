@@ -66,17 +66,20 @@ ABI_VERSION = 2
 
 
 def _build_locked():
-    """Runs build.py (a no-op when the library is newer than every source) under an inter-process file lock: under
-    torchrun all ranks import at once, and only one may compile / link; build.py links to a temporary file and renames."""
+    """Runs build.py under an inter-process file lock when the library is stale: under torchrun all ranks import at
+    once, and only one may compile / link; build.py links to a temporary file and renames. An up-to-date library is
+    loaded without writing anything, so a built tree also works read-only."""
     import fcntl
     import importlib.util
+    spec = importlib.util.spec_from_file_location("_sfcvit_build", os.path.join(_PK, "build.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    if mod.up_to_date():
+        return
     os.makedirs(os.path.dirname(LIB_PATH), exist_ok=True)
     with open(LIB_PATH + ".lock", "w") as lk:
         fcntl.flock(lk, fcntl.LOCK_EX)
         try:
-            spec = importlib.util.spec_from_file_location("_sfcvit_build", os.path.join(_PK, "build.py"))
-            mod = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(mod)
             mod.build()
         finally:
             fcntl.flock(lk, fcntl.LOCK_UN)

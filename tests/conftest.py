@@ -12,14 +12,6 @@ for p in (ROOT, PK, os.path.join(ROOT, "tests", "golden")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200); run with -m gpu")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference mounted (build container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir("/root/reference/src")
-    for item in items:
-        if "needs_reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not mounted"))
 
 
 @pytest.fixture(scope="session")

@@ -1,7 +1,7 @@
 """Import the live reference (/root/reference) under the alias ``refsrc`` (SURVEY.md §8c recipe).
 
 Only usable in the build container (the GPU box has no /root/reference). Used by
-make_golden.py and by tests marked ``needs_reference`` (skipped when the path is absent).
+make_golden.py and make_host_curve_golden.py, which write the fixtures the tests compare against.
 """
 import importlib
 import os
