@@ -44,12 +44,12 @@ struct DropKey {
   uint32_t s0, s1, thr16;
   float inv_keep;
 };
-__device__ __forceinline__ uint32_t drop_thr16(float p) { return (uint32_t)(p * 65536.0f); }
-__device__ __forceinline__ float drop_inv_keep(float p) {
+__host__ __device__ __forceinline__ uint32_t drop_thr16(float p) { return (uint32_t)(p * 65536.0f); }
+__host__ __device__ __forceinline__ float drop_inv_keep(float p) {
   return p > 0.f ? 65536.0f / (65536.0f - (float)drop_thr16(p)) : 1.0f;
 }
-__device__ __forceinline__ DropKey drop_key(unsigned long long seed, float p, const unsigned long long* epoch = nullptr) {
-  if (epoch != nullptr) seed += __ldg(epoch) * 0xD1B54A32D192ED03ull;   // CUDA-graph replays: fresh masks per replay
+// The seed mixing of drop_key without the device-side epoch load (host-callable: tests/host/dropout_host.cu).
+__host__ __device__ __forceinline__ DropKey drop_key_mixed(unsigned long long seed, float p) {
   unsigned long long z = seed + 0x9E3779B97F4A7C15ull;
   z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
   z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
@@ -61,7 +61,14 @@ __device__ __forceinline__ DropKey drop_key(unsigned long long seed, float p, co
   k.inv_keep = drop_inv_keep(p);
   return k;
 }
-__device__ __forceinline__ uint32_t drop_hash2(const DropKey& k, unsigned long long pair) {
+__host__ __device__ __forceinline__ unsigned long long drop_epoch_seed(unsigned long long seed, unsigned long long epoch) {
+  return seed + epoch * 0xD1B54A32D192ED03ull;
+}
+__device__ __forceinline__ DropKey drop_key(unsigned long long seed, float p, const unsigned long long* epoch = nullptr) {
+  if (epoch != nullptr) seed = drop_epoch_seed(seed, __ldg(epoch));   // CUDA-graph replays: fresh masks per replay
+  return drop_key_mixed(seed, p);
+}
+__host__ __device__ __forceinline__ uint32_t drop_hash2(const DropKey& k, unsigned long long pair) {
   uint32_t x = ((uint32_t)pair ^ k.s0) * 0x9E3779B1u;
   x ^= x >> 15;
   x = (x + (uint32_t)(pair >> 32) * 0x632BE5ABu + k.s1) * 0x85EBCA77u;
@@ -79,7 +86,7 @@ __host__ __device__ constexpr uint32_t lcg_mul(int n) { uint32_t a = 1u; for (in
 __host__ __device__ constexpr uint32_t lcg_add(int n) { uint32_t c = 0u; for (int i = 0; i < n; ++i) c = c * kLcgA + kLcgC; return c; }
 
 template <int G>
-__device__ __forceinline__ bool drop_keep(const DropKey& k, unsigned long long idx) {
+__host__ __device__ __forceinline__ bool drop_keep(const DropKey& k, unsigned long long idx) {
   const uint32_t seed = drop_hash2(k, idx / G);
   uint32_t x = seed;
   const int pos = (int)(idx % G);
