@@ -18,7 +18,6 @@
 #include "common.cuh"
 #include "gemm_epilogue.cuh"   // DropKey, drop_apply
 #include "sfcvit.h"
-#include <stdlib.h>
 
 namespace {
 
@@ -77,6 +76,7 @@ __device__ __forceinline__ void store_p_half(uint32_t buf, int r, int c16, const
 // The key tile size is a runtime value (any multiple of 16 up to 208): N <= 208 (the 14 x 14 grid: 196 -> 208) is a
 // single pass without online-softmax rescaling; longer sequences use equal tiles of <= 192 keys, double buffered.
 constexpr int kFwdThreads = 384;
+constexpr int kFwdMaxSingleN = 208;   // longest sequence served in one key pass: the 14 x 14 grid's 196 keys padded to 208
 
 struct FwdLayout {          // runtime shared-memory map (bytes), all tile bases 1024-byte aligned
   int bkv, nkv, stages, p_atoms;
@@ -85,8 +85,7 @@ struct FwdLayout {          // runtime shared-memory map (bytes), all tile bases
 
 inline FwdLayout fwd_layout(int N) {
   FwdLayout L;
-  static const int max_single = getenv("SFC_ATTN_FWD_MAXSINGLE") ? atoi(getenv("SFC_ATTN_FWD_MAXSINGLE")) : 208;   // tuning knob
-  if (N <= max_single) { L.bkv = (N + 15) / 16 * 16; L.nkv = 1; L.stages = 1; }
+  if (N <= kFwdMaxSingleN) { L.bkv = (N + 15) / 16 * 16; L.nkv = 1; L.stages = 1; }
   else {
     L.nkv = (N + 191) / 192;
     if (L.nkv < 2) L.nkv = 2;
@@ -1181,8 +1180,7 @@ extern "C" int sfc_attn_bwd(const void* qkv, const void* out, const void* dout, 
   p.B = B; p.H = H; p.N = N; p.D = D; p.scale = scale; p.drop_p = drop_p; p.drop_seed = drop_seed; p.drop_epoch = sfc_dropout_epoch_ptr();
   p.lse = const_cast<float*>(lse); p.o = (const __nv_bfloat16*)out; p.dout = (const __nv_bfloat16*)dout;
   p.dqkv = (__nv_bfloat16*)dqkv; p.dq_acc = (float*)scratch; p.dq_part = (__nv_bfloat16*)scratch; p.dq_mode = dq_mode;
-  static const bool no_wide = getenv("SFC_ATTN_NO256") != nullptr;          // measurement switch
-  p.wide_st = (!no_wide && ((reinterpret_cast<uintptr_t>(dqkv) | reinterpret_cast<uintptr_t>(scratch)) & 31) == 0) ? 1 : 0;
+  p.wide_st = (((reinterpret_cast<uintptr_t>(dqkv) | reinterpret_cast<uintptr_t>(scratch)) & 31) == 0) ? 1 : 0;
   p.delta = delta; p.dbg = g_attn_dbg;
   static bool configured = false;
   if (!configured) {

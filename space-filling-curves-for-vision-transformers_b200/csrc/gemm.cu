@@ -16,7 +16,6 @@
 #include "common.cuh"
 #include "gemm_epilogue.cuh"
 #include "sfcvit.h"
-#include <stdlib.h>
 #include <string.h>
 
 namespace {
@@ -435,9 +434,8 @@ extern "C" size_t sfc_gemm_workspace_bytes(int M, int N, int K, int splits) {
 static int gemm_pick_bn(int N, int K) {
   if (N <= 128) return 128;
   if (K < 256) return 256;     // very short K (ViT-Tiny, K = 192): per-tile fixed costs dominate, fewer larger tiles win (measured)
-  static const bool off = getenv("SFC_GEMM_BN256") != nullptr;
   const long long pad256 = (long long)sfc_ceil_div(N, 256) * 256, pad128 = (long long)sfc_ceil_div(N, 128) * 128;
-  return (!off && pad128 < pad256 && pad256 * 100 > (long long)N * 115) ? 128 : 256;
+  return (pad128 < pad256 && pad256 * 100 > (long long)N * 115) ? 128 : 256;
 }
 
 // Split count for a GEMM that also returns the row sums of A over K (ep->colsum_out; wgrad: the bias gradient) inside
@@ -446,8 +444,6 @@ static int gemm_pick_bn(int N, int K) {
 extern "C" int sfc_gemm_colsum_splits(int M, int N, int K, int a_mn_major, int b_mn_major) {
   if (!a_mn_major || !b_mn_major) return 0;
   if (sfc_ceil_div(M, BM) < 2 || sfc_ceil_div(K, BK) < 2 || N % 32 != 0 || N < 32) return 0;
-  static const bool off = getenv("SFC_GEMM_NOCOLSUM") != nullptr;
-  if (off) return 0;
   const int s = sfc_gemm_suggest_splits(M, N, K);
   return s < 2 ? 2 : s;
 }
@@ -499,8 +495,6 @@ extern "C" int sfc_gemm_bf16(const void* A, int a_mn_major, long long lda, const
   e.ld_out = ep->ld_out; e.ld_res = ep->ld_res; e.ld_aux = ep->ld_aux;
   e.alpha = ep->alpha;
   e.act = ep->act; e.aux_mode = ep->aux_mode; e.out_fp32 = ep->out_fp32;
-  static const bool no_wide = getenv("SFC_GEMM_NO256") != nullptr;         // measurement switch
-  e.wide_st256 = no_wide ? 0 : 1;
   e.drop_p = ep->drop_p; e.drop_seed = ep->drop_seed; e.drop_epoch = sfc_dropout_epoch_ptr();
   e.split_stride = 0;
   SFC_REQUIRE(e.aux_mode == SFC_AUX_NONE || e.aux != nullptr, "sfc_gemm_bf16: aux_mode set but aux is null");
@@ -530,16 +524,14 @@ extern "C" int sfc_gemm_bf16(const void* A, int a_mn_major, long long lda, const
   }
 
   const bool fast = epi_fast_ok(pk.epi);
-  static const bool cl_off = getenv("SFC_GEMM_NOCLUSTER") != nullptr;
-  const bool cl2 = fast && !cl_off && p.num_m_tiles >= 2;      // CTA pairs, tcgen05.mma.cta_group::2
-  if (want_cs) SFC_REQUIRE(fast && cl2, "sfc_gemm_bf16: colsum_out: operands must be 16-byte aligned (fast epilogue) and CTA pairs enabled");
-  static const bool tma_off = getenv("SFC_GEMM_NOTMASTORE") != nullptr;
+  const bool cl2 = fast && p.num_m_tiles >= 2;      // CTA pairs, tcgen05.mma.cta_group::2
+  if (want_cs) SFC_REQUIRE(fast, "sfc_gemm_bf16: colsum_out: operands must be 16-byte aligned (fast epilogue)");
   // bf16 output: staged in swizzled smem boxes and stored by TMA (EPI 2); one [M, N] operand (residual or ReLU-mask
   // source) is fetched by TMA the same way (EPI 3 / 4). fp32 output (split-K partials) and residual + aux together keep
   // the transposed epilogue.
   const bool has_res = pk.epi.residual != nullptr, has_aux = pk.epi.aux_mode != SFC_AUX_NONE;
   int epi_mode = fast ? 1 : 0;
-  if (fast && !tma_off && !pk.epi.out_fp32 && !(has_res && has_aux)) epi_mode = has_res ? 3 : (has_aux ? 4 : 2);
+  if (fast && !pk.epi.out_fp32 && !(has_res && has_aux)) epi_mode = has_res ? 3 : (has_aux ? 4 : 2);
   CUtensorMap ta, tb, tout, topnd;
   memset(&tout, 0, sizeof(tout));
   memset(&topnd, 0, sizeof(topnd));

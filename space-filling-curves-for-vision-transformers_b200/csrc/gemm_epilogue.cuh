@@ -23,7 +23,6 @@ struct EpiParams {
   int act;                        // SFC_ACT_*
   int aux_mode;                   // SFC_AUX_*
   int out_fp32;
-  int wide_st256;                 // allow 256-bit stores where the addresses are 32-byte aligned (host switch; 0 = off)
   float drop_p;                   // dropout prob applied after activation (0 = off)
   unsigned long long drop_seed;
   const unsigned long long* drop_epoch;   // optional device counter mixed into the seed (null = none)
@@ -360,7 +359,7 @@ __device__ __forceinline__ void epi_tile_fast(const EpiParams& p, uint32_t taddr
   const bool has_bias = p.bias != nullptr, has_res = p.residual != nullptr, has_aux = p.aux_mode != SFC_AUX_NONE;
   const bool has_drop = p.drop_p > 0.0f, f32 = p.out_fp32 != 0;
   // fp32 output (split-K partials): two 16-byte stores per lane would each half-fill 32 sectors per instruction
-  const bool wide_f32 = f32 && p.wide_st256 && (reinterpret_cast<uintptr_t>(p.out) & 31) == 0 && p.ld_out % 8 == 0 && p.split_stride % 8 == 0 &&
+  const bool wide_f32 = f32 && (reinterpret_cast<uintptr_t>(p.out) & 31) == 0 && p.ld_out % 8 == 0 && p.split_stride % 8 == 0 &&
                         n_begin % 8 == 0;
   const float relu_lo = p.act == SFC_ACT_RELU ? 0.0f : -INFINITY;
   const float alpha = p.alpha;

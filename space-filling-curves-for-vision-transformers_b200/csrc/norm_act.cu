@@ -377,9 +377,7 @@ extern "C" int sfc_layernorm_bwd(const void* dy, const void* x, const float* mea
   FinalizeOut outs;
   outs.ptr[0] = dgamma; outs.ptr[1] = dbeta; outs.ptr[2] = dcolsum;
   dim3 grid(sfc_ceil_div(D, 32), csum ? 3 : 2);
-  static const bool fin8 = getenv("SFC_FIN8") != nullptr;                 // measurement switch: the 8-lane variant
-  if (fin8) SFC_CUDA_OK(sfc_launch_pdl(partial_finalize_kernel<8>, grid, dim3(256), 0, stream, (const float*)scratch, blocks, 3ll * D, (long long)D, D, outs, param_fp32, accumulate));
-  else SFC_CUDA_OK(sfc_launch_pdl(partial_finalize_kernel<32>, grid, dim3(1024), 0, stream, (const float*)scratch, blocks, 3ll * D, (long long)D, D, outs, param_fp32, accumulate));
+  SFC_CUDA_OK(sfc_launch_pdl(partial_finalize_kernel<32>, grid, dim3(1024), 0, stream, (const float*)scratch, blocks, 3ll * D, (long long)D, D, outs, param_fp32, accumulate));
   SFC_LAUNCH_OK();
   return 0;
 }

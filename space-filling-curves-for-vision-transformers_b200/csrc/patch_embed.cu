@@ -19,7 +19,6 @@
 #include "common.cuh"
 #include "gemm_epilogue.cuh"
 #include "sfcvit.h"
-#include <stdlib.h>
 
 namespace {
 
@@ -35,7 +34,7 @@ struct PatchParams {
   const int* perm;       // [ntok * g] flat pre-patch index r*gw + c in curve order
   int B, C, H, W, p, g, gw;
   int in_fmt;            // SFC_IMG_F32_NCHW / SFC_IMG_BF16_NCHW / SFC_IMG_U8_NHWC
-  int dual_epi;          // single-k-block tiles: the second producer group converts the upper column half (see kernel)
+  int dual_epi;          // always 1: a runtime operand of the kernel's `dual` test (see patch_embed_fwd_kernel)
   int wide_ld, wide_st;  // 256-bit accesses: fp32 chunk = one 32-byte load (image 32-byte aligned), output rows 32-byte aligned
   int row_split;         // p == 4 (NCHW): an 8-element chunk is two 4-element patch rows, the second `row_split` (= W)
                          // elements after the first; 0 = the chunk is one contiguous run
@@ -262,6 +261,9 @@ patch_embed_fwd_kernel(const __grid_constant__ CUtensorMap tmap_w, const PatchPa
   // One k-block per tile (K <= 64: /4 pre-patches of small images): a tile costs one gather round but a full-width
   // epilogue, so the second producer group converts the upper half of the tile's columns instead of idling
   // (ViT-Tiny/4, B = 8192, same box: 0.198 -> 0.160 ms).
+  // pp.dual_epi is always 1, but testing it keeps ptxas's register allocation of the row-per-lane epilogue: with `dual`
+  // derived from num_k_blocks alone the FAST_EPI instantiations spill 48 / 60 bytes instead of 28 / 40, inside the
+  // chunk loop, and bf16 ViT-Tiny/4 (B = 8192) slows from 0.110 to 0.127 ms (B200, 1000 W).
   const bool dual = FAST_EPI && pp.num_k_blocks == 1 && pp.dual_epi != 0;
   if constexpr (VEC) build_chunk_table(pp, tbl, tblq);
 
@@ -743,12 +745,10 @@ int fill_params(PatchParams& pp, const void* img, int img_bf16, int B, int C, in
               "patch_embed: unknown image format %d", img_bf16);
   pp.in_fmt = img_bf16;
   pp.row_split = (img_bf16 != SFC_IMG_U8_NHWC && p == 4) ? W : 0;
-  static const bool no_wide = getenv("SFC_PE_NO256") != nullptr;               // measurement switch
   // fp32 chunks as single 32-byte loads: every chunk offset is a multiple of 8 floats when the vectorised path applies
-  pp.wide_ld = (!no_wide && img_bf16 == SFC_IMG_F32_NCHW && p % 8 == 0 && (reinterpret_cast<uintptr_t>(img) & 31) == 0) ? 1 : 0;
+  pp.wide_ld = (img_bf16 == SFC_IMG_F32_NCHW && p % 8 == 0 && (reinterpret_cast<uintptr_t>(img) & 31) == 0) ? 1 : 0;
   pp.wide_st = 0;
-  static const int dual_env = getenv("SFC_PE_DUAL") ? atoi(getenv("SFC_PE_DUAL")) : 1;      // 0: measurement switch
-  pp.dual_epi = dual_env;
+  pp.dual_epi = 1;
   SFC_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0 && p > 0 && g > 0 && D > 0, "patch_embed: bad shape");
   SFC_REQUIRE(H % p == 0 && W % p == 0, "patch_embed: image %dx%d not divisible by pre-patch size %d", H, W, p);
   const int gh = H / p, gw = W / p;
@@ -798,11 +798,11 @@ extern "C" int sfc_patch_embed_fwd(const void* img, int img_bf16, int B, int C, 
   pp.rows_per_img = rows_per_img; pp.tok_off = tok_off;
   const int BN = (D > 128) ? 256 : 128;
   pp.num_n_tiles = sfc_ceil_div(D, BN);
-  pp.wide_st = (getenv("SFC_PE_NO256") == nullptr && (reinterpret_cast<uintptr_t>(out) & 31) == 0 && (ld_out * 2) % 32 == 0 && D % 16 == 0) ? 1 : 0;
+  pp.wide_st = ((reinterpret_cast<uintptr_t>(out) & 31) == 0 && (ld_out * 2) % 32 == 0 && D % 16 == 0) ? 1 : 0;
   EpiParams& e = pp.epi;
   e.N = D; e.bias = (const __nv_bfloat16*)bias; e.residual = (const __nv_bfloat16*)pos; e.aux = nullptr;
   e.out = out; e.out_pre = nullptr; e.ld_out = ld_out; e.ld_res = ld_pos; e.ld_aux = 0; e.split_stride = 0;
-  e.alpha = 1.0f; e.act = SFC_ACT_NONE; e.aux_mode = SFC_AUX_NONE; e.out_fp32 = 0; e.wide_st256 = 0; e.drop_p = 0.f; e.drop_seed = 0; e.drop_epoch = nullptr;
+  e.alpha = 1.0f; e.act = SFC_ACT_NONE; e.aux_mode = SFC_AUX_NONE; e.out_fp32 = 0; e.drop_p = 0.f; e.drop_seed = 0; e.drop_epoch = nullptr;
   CUtensorMap tw;
   if (int err = sfc_make_tmap_2d(&tw, Wk, 2, (uint64_t)pp.Kpad, (uint64_t)D, (uint64_t)pp.Kpad * 2, BK, (uint32_t)BN, true)) return err;
   // the fused kernels take one pre-patch origin per 64-element k-block: p == 4 (48 elements per pre-patch at C = 3) only for g == 1
@@ -810,18 +810,16 @@ extern "C" int sfc_patch_embed_fwd(const void* img, int img_bf16, int B, int C, 
   const bool u8 = img_bf16 == SFC_IMG_U8_NHWC;
   SFC_REQUIRE(!u8 || vec, "sfc_patch_embed_fwd: uint8 NHWC input with K = %d exceeds the chunk table", pp.K);
   const bool fast = epi_fast_ok(pp.epi);
-  static const bool tm_off = getenv("SFC_PE_NOTMEM") != nullptr;
-  if (vec && pp.row_split == 0 && fast && !tm_off && pp.num_k_blocks <= kTmMaxKb && D % (2 * kTmBN) == 0 && D <= kTmMaxD) {
+  if (vec && pp.row_split == 0 && fast && pp.num_k_blocks <= kTmMaxKb && D % (2 * kTmBN) == 0 && D <= kTmMaxD) {
     // TMEM-resident A: gather once per token, 64-column passes over the weights
     pp.num_n_tiles = D / kTmBN;
-    static const int cl = getenv("SFC_PE_CLUSTER") ? atoi(getenv("SFC_PE_CLUSTER")) : 4;
 #define PE_TMEM(CL_)                                                                            \
   do {                                                                                          \
     if (u8) return launch_pe_tmem<IN_U8, CL_>(Wk, D, pp, stream);                               \
     return img_bf16 ? launch_pe_tmem<IN_BF16, CL_>(Wk, D, pp, stream) : launch_pe_tmem<IN_F32, CL_>(Wk, D, pp, stream); \
   } while (0)
-    if (cl == 4 && pp.num_m_tiles >= 4) PE_TMEM(4);
-    if (cl >= 2 && pp.num_m_tiles >= 2) PE_TMEM(2);
+    if (pp.num_m_tiles >= 4) PE_TMEM(4);
+    if (pp.num_m_tiles >= 2) PE_TMEM(2);
     PE_TMEM(1);
 #undef PE_TMEM
   }

@@ -287,18 +287,6 @@ def test_gemm_epilogue_mask_is_the_reference_ncols_odd(cuda_device, M, N):
     _gemm_case(M, N, "ncols_odd", seed=17 + M + N)
 
 
-@pytest.mark.parametrize("env", [{"SFC_GEMM_NOTMASTORE": "1"}, {"SFC_GEMM_NOCLUSTER": "1"}])
-def test_gemm_epilogue_mask_env_variants(cuda_device, env):
-    """The env switches are read once per process (TMA store off: EPI 1 for bf16; CTA pairs off), so each runs in a child."""
-    code = ("import sys; sys.path[:0] = ['tests', 'space-filling-curves-for-vision-transformers_b200']; "
-            "import test_gpu_dropout as t\n"
-            "for M in (100, 300):\n"
-            "    for N in (640, 768):\n"
-            "        for v in ('plain', 'res', 'aux', 'fp32'):\n"
-            "            t._gemm_case(M, N, v, seed=M + N + 3)\n")
-    subprocess.run([sys.executable, "-c", code], cwd=ROOT, env={**os.environ, **env}, check=True, timeout=300)
-
-
 # ------------------------------------------------------------------------------------------------- act_bwd / layernorm_bwd
 @pytest.mark.parametrize("n", [8 * 1000 + 8, 4096 * 3 + 72])           # multiples of 8, not of 64
 @pytest.mark.parametrize("mode", ["none", "gelu_grad", "relu_mask"])
